@@ -46,6 +46,7 @@ import numpy as np
 
 ROOT = Path(__file__).resolve().parent
 sys.path.insert(0, str(ROOT))
+sys.dont_write_bytecode = True          # the benchmark leaves the tree it runs from as it found it (it may be read-only)
 
 SEED = 0x4C6F5202
 METRIC = "LoRa symbols/s (dechirp+FFT+argmax)"
@@ -66,6 +67,8 @@ def parse_args():
     ap.add_argument("--no-config4", action="store_true")
     ap.add_argument("--no-cpu", action="store_true")
     ap.add_argument("--cpu-seconds", type=float, default=12.0)
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the timed path's outputs of its last step (bins.npy, mags.npy, float32) to DIR")
     return ap.parse_args()
 
 
@@ -379,6 +382,23 @@ K1_KERNEL = {7: "k1_sf7_warp_kernel<12,2>", 8: "k1_group_kernel<8,6,2>", 9: "k1_
              11: "k1_rows_kernel<11>", 12: "k1_rows_kernel<12>"}
 
 
+DUMP_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir: Path, bins, mags):
+    """What a caller of demod_fft receives from the last timed step: bins.npy and mags.npy (float32; a bin < 2^12 is exact).
+    The inputs follow from SEED and the arguments alone, so two builds run with the same arguments can be compared output
+    for output.  A batch above DUMP_BYTES is sampled at fixed, seeded symbol indices, written as index.npy (float64)."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    b, m = bins.cpu().numpy().astype(np.float32), mags.cpu().numpy().astype(np.float32)
+    if b.nbytes + m.nbytes > DUMP_BYTES:
+        idx = np.sort(np.random.default_rng(SEED).choice(b.size, DUMP_BYTES // 16, replace=False))
+        b, m = b[idx], m[idx]
+        np.save(out_dir / "index.npy", idx.astype(np.float64))
+    np.save(out_dir / "bins.npy", b)
+    np.save(out_dir / "mags.npy", m)
+
+
 def run_reference(args):
     """--impl reference: the reference's CPU get_shift_fft on all host threads it may use; rank 0 only."""
     rank = int(os.environ.get("RANK", "0"))
@@ -503,6 +523,8 @@ def main():
     if world > 1:
         dist.barrier()
     launches = dec.launch_count() - l0
+    if args.dump_outputs and rank == 0:
+        dump_outputs(Path(args.dump_outputs), bins, mags)      # before the per-SF table below reuses the buffers
     ms = e0.elapsed_time(e1)
     ms_max = all_max(ms)
     clocks = sampler.stop(t0, t1) if rank == 0 else None

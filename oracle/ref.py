@@ -26,9 +26,16 @@ REF_ROOT = Path("/root/reference")
 _lib = None
 
 
+def _have_sources() -> bool:
+    try:
+        return (REF_ROOT / "lib" / "decoder_impl.cc").is_file()
+    except OSError:          # a directory the user may not enter: the sources are absent for this user
+        return False
+
+
 def build(force: bool = False) -> Path | None:
     """(Re)build where the reference sources exist; otherwise keep whatever prebuilt file travelled here."""
-    if (REF_ROOT / "lib" / "decoder_impl.cc").exists():
+    if _have_sources():
         if force and LIB.exists():
             LIB.unlink()
         subprocess.run(["make", "-C", str(HERE), "-s", "ref"], check=True)
@@ -36,7 +43,7 @@ def build(force: bool = False) -> Path | None:
 
 
 def available() -> bool:
-    return LIB.exists() or (REF_ROOT / "lib" / "decoder_impl.cc").exists()
+    return LIB.exists() or _have_sources()
 
 
 def lib():

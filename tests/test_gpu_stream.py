@@ -184,7 +184,8 @@ def test_other_sample_rates_gradient_path(torch, oracle, fs):
 def test_cfo_estimate_equals_reference_function(torch, oracle, ref, cfo_hz):
     """N4: lora_b200_set_cfo_estimate -> experimental_determine_cfo (lib/decoder_impl.cc:730-738) at the SYNC step, on the
     window the reference's commented-out call site would pass (&input[i], :774).  Compared with the reference's own
-    function (oracle/_ref); frames and the step trace are untouched by the option."""
+    function (oracle/_ref, its recorded answers: tests/golden/refcalls.py); frames and the step trace are untouched by the
+    option."""
     import gr_lora_b200 as G
     from conftest import make_capture
     x = make_capture(bytes.fromhex("0123456789abcdef"), 8, 4, True, seed=33, cfo_hz=cfo_hz)
