@@ -23,6 +23,17 @@ class Step(C.Structure):
                 ("metric", C.c_float)]
 
 
+class GatewayConfig(C.Structure):
+    """struct lora_b200_gateway_config (include/lora_b200.h)."""
+    _fields_ = [
+        ("samp_rate", C.c_float), ("center_freq", C.c_float), ("channel_list", C.POINTER(C.c_float)),
+        ("n_channels", C.c_uint32), ("bandwidth", C.c_uint32), ("decimation", C.c_uint32), ("sf_mask", C.c_uint32),
+        ("reduced_rate_mask", C.c_uint32), ("implicit", C.c_uint8), ("cr", C.c_uint8), ("crc", C.c_uint8), ("demod", C.c_uint8),
+        ("conj", C.c_uint8), ("disable_drift_correction", C.c_uint8), ("reserved", C.c_uint8 * 2), ("device", C.c_int32),
+        ("max_in_per_call", C.c_uint32), ("max_frames_per_call", C.c_uint32),
+    ]
+
+
 FRAME_CB = C.CFUNCTYPE(None, C.c_void_p, C.c_uint32, C.POINTER(C.c_uint8), C.c_size_t)
 
 OK, EINVAL, ECUDA, ENOMEM, EUNSUPPORTED, EOVERFLOW = 0, -1, -2, -3, -4, -5
@@ -81,6 +92,13 @@ SIGNATURES = {
     "lora_b200_channelizer_output": (_vp, [_vp, _u32, C.POINTER(_sz)]),
     "lora_b200_channelizer_read_output": (_i, [_vp, _u32, _vp, _sz]),
     "lora_b200_channelizer_launch_count": (C.c_uint64, [_vp]),
+    "lora_b200_gateway_create": (_vp, [C.POINTER(GatewayConfig)]),
+    "lora_b200_gateway_destroy": (None, [_vp]),
+    "lora_b200_gateway_reset": (_i, [_vp]),
+    "lora_b200_gateway_work": (_i, [_vp, _vp, _sz, _i, C.POINTER(_sz)]),
+    "lora_b200_gateway_frames_last": (_sz, [_vp, C.POINTER(_vp)]),
+    "lora_b200_gateway_position": (_i, [_vp, _u32, _u32, C.POINTER(C.c_uint64), C.POINTER(C.c_uint32)]),
+    "lora_b200_gateway_timing": (_i, [_vp, C.POINTER(C.c_float), _sz]),
 }
 
 _lib = None

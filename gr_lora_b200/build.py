@@ -37,7 +37,7 @@ def _sources():
     return sorted(CSRC.glob("*.cu")) + sorted(CSRC.glob("*.cuh")) + sorted(CSRC.glob("*.h")) + [ROOT / "include" / "lora_b200.h"]
 
 
-TRANSLATION_UNITS = ("lora_b200.cu", "k1_rows.cu", "k1_packed.cu", "channelizer.cu")
+TRANSLATION_UNITS = ("lora_b200.cu", "k1_rows.cu", "k1_packed.cu", "channelizer.cu", "gateway.cu")
 
 
 def build(force: bool = False, verbose: bool = False) -> Path:

@@ -8,6 +8,7 @@
 #include "k1_rows.cuh"
 #include "int_chain.cuh"
 #include "tx_channel.cuh"
+#include "gateway_gather.cuh"
 
 extern "C" {
 
@@ -78,5 +79,21 @@ uint8_t lb_emul_hamming84_decode(uint8_t cw) { return lb::hamming84_decode(cw); 
 uint8_t lb_emul_hamming84_encode(uint8_t v) { return lb::hamming84_encode(v); }
 uint8_t lb_emul_deshuffle(uint8_t v) { return lb::deshuffle_byte(v); }
 int32_t lb_emul_payload_symbols(uint32_t len, uint32_t cr, uint32_t sf, int rr) { return lb::payload_symbols(len, cr, sf, rr); }
+
+// the gateway's gather (gateway_gather.cuh) on the host: next[0, pending + m) from prev's tail and o, element by element
+// through the kernel's index map; returns the new length, or -1 (next untouched) when it would exceed cap
+int64_t lb_emul_gw_gather(const float2 *prev, uint32_t consumed, uint32_t pending, const float2 *o, uint32_t m, uint32_t cap,
+                          float2 *next) {
+    int ovf = 0;
+    const uint32_t n = lb::gw_next_len(pending, m, cap, &ovf);
+    if (ovf) return -1;
+    for (uint32_t i = 0; i < n; i++) {
+        int fp;
+        const uint32_t s = lb::gw_src(i, consumed, pending, &fp);
+        next[i] = fp ? prev[s] : o[s];
+    }
+    return n;
+}
+uint32_t lb_emul_gw_pending(uint32_t len, uint32_t consumed) { return lb::gw_pending(len, consumed); }
 
 }

@@ -12,6 +12,7 @@
 #include "tx_channel.cuh"
 #include "k1_rows.h"
 #include "k1_packed.h"
+#include "rx_internal.h"
 
 #include <algorithm>
 #include <cmath>
@@ -403,11 +404,13 @@ int rx_begin(lora_b200_decoder *d) {
 }
 
 // the state machine for streams [stream_base, stream_base + n_launch) over staged IQ (one CTA per stream), async on rx_stream
+// (n_items_s: per-stream item counts on the device, indexed by stream; nullptr = n_items for all)
 int rx_launch(lora_b200_decoder *d, const float2 *d_iq, size_t stride_items, size_t n_items, uint32_t stream_base, uint32_t n_launch,
-              cudaStream_t st = nullptr) {
+              cudaStream_t st = nullptr, const uint32_t *n_items_s = nullptr) {
     RxParams p;
     memset(&p, 0, sizeof p);
-    p.iq = d_iq; p.stride_items = stride_items; p.n_items = n_items; p.stream_base = stream_base; p.n_launch = n_launch;
+    p.iq = d_iq; p.stride_items = stride_items; p.n_items = n_items; p.n_items_s = n_items_s;
+    p.stream_base = stream_base; p.n_launch = n_launch;
     p.down = tab<float2>(d, d->toff.down);
     p.down_ifreq = tab<float>(d, d->toff.down_ifreq);
     p.up_ifreq = tab<float>(d, d->toff.up_ifreq);
@@ -517,6 +520,31 @@ __global__ void sc8_to_cf32_kernel(const char2 *__restrict__ in, float2 *__restr
 }
 
 }  // namespace
+
+// ---- internal entry points for gateway.cu (rx_internal.h) ---------------------------------------
+int lb_fail(int code, const char *fmt, ...) {
+    char buf[512];
+    va_list ap;
+    va_start(ap, fmt);
+    vsnprintf(buf, sizeof buf, fmt, ap);
+    va_end(ap);
+    return fail(code, "%s", buf);
+}
+
+int lb_rx_launch_streams(lora_b200_decoder *d, const float2 *iq, size_t stride_items, const uint32_t *n_items_s, cudaEvent_t ready,
+                         cudaEvent_t done) {
+    CU(cudaSetDevice(d->device));
+    CU(cudaStreamWaitEvent(d->rx_stream, ready, 0));
+    int rc = rx_begin(d);
+    if (!rc) rc = rx_launch(d, iq, stride_items, stride_items, 0, d->cfg.n_streams, d->rx_stream, n_items_s);
+    if (!rc) CU(cudaEventRecord(done, d->rx_stream));
+    return rc;
+}
+
+int lb_rx_finish_streams(lora_b200_decoder *d, size_t *consumed) {
+    CU(cudaSetDevice(d->device));
+    return rx_finish(d, 0, d->cfg.n_streams, consumed, nullptr, nullptr);
+}
 
 // =================================================================================================
 // C ABI

@@ -92,7 +92,12 @@ struct RxParams {
     lora_b200_step *trace;
     uint32_t trace_cap;
     uint32_t *trace_n;                 // per stream
+    const uint32_t *n_items_s;         // per-stream item counts [stream] (device); nullptr: every stream has n_items
 };
+
+// the items stream `stream` may read in this launch (read where it is used rather than held in a register: the kernels
+// are at their register budget)
+#define LB_RX_N_ITEMS(p, stream) ((p).n_items_s ? (unsigned long long)(p).n_items_s[stream] : (unsigned long long)(p).n_items)
 
 #ifdef __CUDACC__
 
@@ -229,7 +234,7 @@ rx_stream_kernel(RxParams p) {
     while (true) {
         const unsigned long long pos = sh.pos;
         const int state = sh.state;
-        if (pos + 2ull * (unsigned long long)sps > p.n_items) break;
+        if (pos + 2ull * (unsigned long long)sps > LB_RX_N_ITEMS(p, stream)) break;
         if (sh.frames_here >= p.max_frames_per_stream) break;
         const float2 *x = xs + pos;
         if (tid == 0) { sh.fine_sync = 0; sh.bin = -1; sh.metric = 0.0f; sh.flag = 0; sh.consumed = 0; }   // :749

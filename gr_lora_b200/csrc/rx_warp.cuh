@@ -280,7 +280,7 @@ rx_warp_kernel(RxParams p) {
     unsigned int frames_here = 0, steps = 0;
 
     while (true) {
-        if (pos + 2ull * (unsigned long long)sps > p.n_items) break;
+        if (pos + 2ull * (unsigned long long)sps > LB_RX_N_ITEMS(p, stream)) break;
         if (frames_here >= p.max_frames_per_stream) break;
         const float2 *x = xs + pos;
         int consumed = 0, fine = 0, bin = -1, next_state = state;     // :749
@@ -335,7 +335,7 @@ rx_warp_kernel(RxParams p) {
             break;
         }
         case LORA_B200_FIND_SFD: {                                // :785-818, A10
-            rw_load(x, win, sps, lane, xs + p.n_items);
+            rw_load(x, win, sps, lane, xs + LB_RX_N_ITEMS(p, stream));
             __syncwarp();
             rw_ifreq<true>(win, ifq, sps, lane);                  // padded: float i at i + (i >> 5) = lane + 33 j for i = lane + 32 j
             const int to_idx = sps - 1;
@@ -377,7 +377,7 @@ rx_warp_kernel(RxParams p) {
         case LORA_B200_DECODE_HEADER:
         case LORA_B200_DECODE_PAYLOAD: {                          // :826-886
             const bool is_first = state == LORA_B200_DECODE_HEADER;
-            rw_load(x, win, sps, lane, xs + p.n_items);
+            rw_load(x, win, sps, lane, xs + LB_RX_N_ITEMS(p, stream));
             __syncwarp();
             bool do_demod = true;
             if (!is_first && p.implicit) {                        // :861 determine_energy

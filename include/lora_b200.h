@@ -242,6 +242,55 @@ const void *lora_b200_channelizer_output(const lora_b200_channelizer *c, uint32_
 int lora_b200_channelizer_read_output(const lora_b200_channelizer *c, uint32_t channel, void *host_dst, size_t n_items);
 uint64_t lora_b200_channelizer_launch_count(const lora_b200_channelizer *c);
 
+/* ---- N4 (SURVEY.md 8f): the gateway receiver -- every channel AND every spreading factor of a wideband capture --------
+ * Wideband IQ in, chunk by chunk; the frames of every (channel, SF) out, one call per chunk, the IQ staying in device
+ * memory.  A call runs the channelizer above over the chunk (the same entry point, so every channel's samples are those a
+ * standalone lora_b200_channelizer fed the same chunks produces), appends each channel's new samples to the items every
+ * SF's decoder left unconsumed in the previous call, and runs one decoder per SF (lora_b200_create with
+ * n_streams = n_channels, samp_rate / decimation) on all channels, the SFs concurrently.  Each (channel, SF) stream decodes
+ * exactly what lora_b200_work on that channel's samples decodes. */
+typedef struct lora_b200_gateway lora_b200_gateway;
+typedef struct lora_b200_gateway_config {
+    float        samp_rate;          /* wideband rate                                                               */
+    float        center_freq;
+    const float *channel_list;       /* n_channels absolute frequencies, as lora_b200_channelizer_create              */
+    uint32_t     n_channels;
+    uint32_t     bandwidth;
+    uint32_t     decimation;         /* decoders run at samp_rate / decimation                                        */
+    uint32_t     sf_mask;            /* bit s set: decode SF s (7..12) on every channel                               */
+    uint32_t     reduced_rate_mask;  /* bit s set: reduced_rate for SF s; 0 = LoRa's default at 125 kHz (SF11, SF12) */
+    uint8_t      implicit, cr, crc, demod;   /* as lora_b200_config, shared by all SFs                               */
+    uint8_t      conj;               /* conjugate on the way out of the FIR bank (lora_receiver conj=True)            */
+    uint8_t      disable_drift_correction;
+    uint8_t      reserved[2];
+    int32_t      device;
+    uint32_t     max_in_per_call;    /* wideband items per call (0 = 1<<22)                                          */
+    uint32_t     max_frames_per_call;/* per (channel, SF) stream (0 = 8)                                              */
+} lora_b200_gateway_config;
+
+typedef struct lora_b200_gateway_frame {
+    uint32_t channel;                /* index into channel_list */
+    uint32_t sf;
+    lora_b200_frame frame;           /* frame.stream == channel */
+} lora_b200_gateway_frame;
+
+/* The arguments are checked before a device is looked for (EINVAL via lora_b200_last_error). */
+lora_b200_gateway *lora_b200_gateway_create(const lora_b200_gateway_config *cfg);
+void lora_b200_gateway_destroy(lora_b200_gateway *g);
+/* decoders AND channelizer history / rotator back to the state of a fresh gateway */
+int lora_b200_gateway_reset(lora_b200_gateway *g);
+/* n_in: a multiple of decimation, <= max_in_per_call; host_ptr as lora_b200_work_batch.  *n_frames = frames decoded.
+ * LORA_B200_EOVERFLOW (nothing consumed, nothing changed): a stream's unconsumed items plus this chunk would not fit its
+ * buffer -- only possible when a stream stopped at max_frames_per_call; a smaller chunk fits. */
+int lora_b200_gateway_work(lora_b200_gateway *g, const void *iq, size_t n_in, int host_ptr, size_t *n_frames);
+/* the frames of the last work call, ordered by (sf ascending, channel, seq); valid until the next call */
+size_t lora_b200_gateway_frames_last(lora_b200_gateway *g, const lora_b200_gateway_frame **frames);
+/* progress of one stream: items consumed since create/reset, and items held over for the next call */
+int lora_b200_gateway_position(lora_b200_gateway *g, uint32_t channel, uint32_t sf, uint64_t *consumed, uint32_t *pending);
+/* where the last work call spent its device time, from CUDA events, in ms: [0] host-to-device copy, [1] channelizer,
+ * [2] gather, [3] the decoders' state machines (all SFs, concurrently) */
+int lora_b200_gateway_timing(const lora_b200_gateway *g, float *ms, size_t n);
+
 /* how many kernels this library has launched since creation (bench.py's gpu_launches) */
 uint64_t lora_b200_launch_count(const lora_b200_decoder *d);
 
